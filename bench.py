@@ -33,6 +33,13 @@ the table fits one GPU); the other one is the sub-record of its name.  Total wor
 --impl reference times the reference's own CPU implementation of the path on a bounded
 sample per step (oracle/_ref = the unmodified torchkge package when present, else the oracle
 port oracle/kge_oracle.py, which tests/golden pins against it).
+
+--dump-outputs DIR writes what the timed path computed in its last timed step as DIR/<name>.npy
+(integers as float64, floating-point results as float32): the four rank vectors of a link-prediction
+workload (rank_heads, rank_tails, filt_rank_heads, filt_rank_tails; with --impl reference, of the
+last step's sample), or for c5 the loss, the relation gradient table and the gradient rows of a
+fixed seeded sample of DUMP_ROWS entities (grad_ent_rows holds their ids).  Inputs are generated
+from --seed, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -44,6 +51,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the source tree may be read-only: nothing is written into it
 
 # stdout carries exactly one JSON line: keep a private handle on it and point fd 1 at stderr, so
 # that NCCL's INFO lines and any library chatter land on stderr
@@ -59,11 +67,20 @@ def emit(record):
     _REAL_STDOUT.flush()
 
 
+def _count(minimum):
+    def parse(text):
+        v = int(text)
+        if v < minimum:
+            raise argparse.ArgumentTypeError("must be >= %d" % minimum)
+        return v
+    return parse
+
+
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=_count(1), default=3, help="timed steps")
+    ap.add_argument("--warmup", type=_count(0), default=3, help="untimed steps before them")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c2")
     ap.add_argument("--cpu-sample", type=int, default=0,
@@ -76,6 +93,8 @@ def parse_args():
     ap.add_argument("--split", default="auto", choices=["auto", "queries", "entities"],
                     help="multi-GPU decomposition reported as the headline value")
     ap.add_argument("--batch", type=int, default=32768, help="c5: positives per training step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (see the module docstring)")
     return ap.parse_args()
 
 
@@ -132,6 +151,33 @@ class ClockSampler:
 
 
 # ----------------------------------------------------------------------------- helpers
+RANK_NAMES = ("rank_heads", "rank_tails", "filt_rank_heads", "filt_rank_tails")
+DUMP_ROWS = 8192                 # c5: entity gradient rows written by --dump-outputs
+DUMP_LIMIT = 64 << 20            # bytes, all files of one --dump-outputs together
+
+
+def dump_rows(n_ent):
+    """The fixed sample of entity rows whose gradients --dump-outputs writes for c5."""
+    g = torch.Generator().manual_seed(0)
+    return torch.randperm(n_ent, generator=g)[:DUMP_ROWS].sort().values
+
+
+def dump_outputs(directory, arrays):
+    """Write each tensor of `arrays` as directory/<name>.npy: integers as float64 (exact below
+    2^53), floating-point values as float32."""
+    import numpy as np
+    host = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu()
+        host[name] = (a.float() if a.is_floating_point() else a.double()).numpy()
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def dist_info():
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -403,13 +449,15 @@ def run_reference(args, rank, world):
     th, tt, tr = (graph[k][:total].cpu() for k in ("test_h", "test_t", "test_r"))
     b_size = 4 if big else 256
     sharded = table_bytes(wl) > 8e9
+    last = {}
     if sharded:
         impl = "port"
 
         def step(i):
             lo, hi = i * per_step, (i + 1) * per_step
-            return oracle_ranks_sharded(kind, code, wl, args.seed, th[lo:hi], tt[lo:hi], tr[lo:hi], dh, dt,
-                                        dev, 8)[1]
+            last["ranks"], s_ = oracle_ranks_sharded(kind, code, wl, args.seed, th[lo:hi], tt[lo:hi], tr[lo:hi],
+                                                     dh, dt, dev, 8)
+            return s_
     else:
         tabs = S.make_tables(code, wl["dim"], wl["n_ent"], wl["n_rel"], 0, wl["n_ent"], args.seed, dev)
         P = oracle_params_from_tables(kind, {k: (v.cpu() if v is not None else None) for k, v in tabs.items()})
@@ -419,7 +467,7 @@ def run_reference(args, rank, world):
         def step(i):
             lo, hi = i * per_step, (i + 1) * per_step
             t0 = time.perf_counter()
-            ref.ranks(th[lo:hi], tt[lo:hi], tr[lo:hi], dh, dt, b_size)
+            last["ranks"] = ref.ranks(th[lo:hi], tt[lo:hi], tr[lo:hi], dh, dt, b_size)
             return time.perf_counter() - t0
 
     for i in range(args.warmup):
@@ -428,6 +476,8 @@ def run_reference(args, rank, world):
     for i in range(args.steps):
         el += step(args.warmup + i)
     value = args.steps * per_step / el
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(RANK_NAMES, last["ranks"])))
     sample = "%d test triples per step (b_size %d) of workload %s%s" % (
         per_step, 1 if sharded else b_size, args.workload,
         ", table scored in 8 entity-range pieces (40 GB does not fit the scorer's temporaries)" if sharded else "")
@@ -460,6 +510,9 @@ def run_reference_c5(args):
     g = torch.Generator().manual_seed(1)
     probs = torch.rand(c5["n_rel"], generator=g) * 0.8 + 0.1
 
+    rows = dump_rows(c5["n_ent"])
+    last = {}
+
     def step():
         h = torch.randint(0, c5["n_ent"], (b,), generator=g)
         t = torch.randint(0, c5["n_ent"], (b,), generator=g)
@@ -469,17 +522,23 @@ def run_reference_c5(args):
         pos, neg = oracle.forward_pos_neg("distmult", P, h, t, r, nh, nt)
         loss = oracle.margin_loss(pos, neg, 1.0)
         loss.backward()
+        el_ = time.perf_counter() - t0
+        if args.dump_outputs:
+            last.update(loss=loss.detach().view(1), grad_ent_rows=rows, grad_ent=P["ent"].grad[rows],
+                        grad_rel=P["rel"].grad.clone())
         for p in P.values():
             p.grad = None
-        return time.perf_counter() - t0
+        return el_
 
-    for _ in range(min(args.warmup, 1)):
+    for _ in range(args.warmup):
         step()
-    steps = min(args.steps, 3)
+    steps = args.steps
     el = sum(step() for _ in range(steps))
     value = steps * b / el
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     emit({"impl": "reference", "metric": C5_METRIC, "value": value, "unit": "positives/s", "n_gpus": args.gpus,
-          "steps": steps, "warmup": min(args.warmup, 1), "ms_per_step": 1000 * el / steps,
+          "steps": steps, "warmup": args.warmup, "ms_per_step": 1000 * el / steps,
           "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
           "config": {"workload": c5_workload_text(b)},
           "cpu_baseline": {"value": value, "unit": "positives/s", "cores": cores, "kind": "port",
@@ -813,6 +872,8 @@ def run_ours(args, rank, local, world):
     for mode in modes[1:]:
         out[mode] = recs[mode]
     out.update(extras)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(RANK_NAMES, main_ranks)))
     emit(out)
     if world > 1:
         dist.destroy_process_group()
@@ -869,10 +930,12 @@ def c5_workload_text(b):
             % (c5["dim"], c5["n_ent"], c5["n_rel"], b, c5["n_neg"]))
 
 
-def measure_c5(args, dev, cpu_steps=1, batches=(4096, 32768)):
+def measure_c5(args, dev, cpu_steps=1, batches=(4096, 32768), reps=None, warm=3, outputs=None):
     """C5 (BASELINE.json configs[4]) on one GPU: forward and forward+backward of the fused step,
     HBM roofline on SURVEY.md section 8d's algorithmic bytes ((n_neg + 3) * 4d forward, x3 with
-    backward, per positive), parity with supplied negatives against the oracle, CPU baseline."""
+    backward, per positive), parity with supplied negatives against the oracle, CPU baseline.
+    `reps` timed and `warm` untimed calls of each form (reps None: --steps clamped to [3, 10]);
+    `outputs`, a dict, receives what the last timed forward+backward at batches[-1] computed."""
     import torchkge_b200 as tk
     from torchkge_b200 import synthetic as S
     from torchkge_b200.training import fused_margin_step
@@ -893,6 +956,7 @@ def measure_c5(args, dev, cpu_steps=1, batches=(4096, 32768)):
     row = 4 * dim
     out = {"workload": c5_workload_text(batches[-1]), "metric": C5_METRIC, "by_batch": {}}
     calls = [0]
+    last = {}
 
     def timed(fn, reps, warm=3):
         for _ in range(warm):
@@ -923,6 +987,7 @@ def measure_c5(args, dev, cpu_steps=1, batches=(4096, 32768)):
                 p.grad = None
             loss = fused_margin_step(model, h, t, r, 1.0, n_neg=n_neg, bern_probs=probs, seed=7, offset=calls[0])
             loss.backward()
+            last["loss"] = loss
             return loss
 
         def e2e_step():
@@ -935,8 +1000,14 @@ def measure_c5(args, dev, cpu_steps=1, batches=(4096, 32768)):
             loss.backward()
             return loss.item()
 
-        reps = max(3, min(args.steps, 10))
-        ms_f, ms_fb = timed(fwd, reps), timed(fwd_bwd, reps)
+        if reps is None:
+            reps = max(3, min(args.steps, 10))
+        ms_f, ms_fb = timed(fwd, reps, warm), timed(fwd_bwd, reps, warm)
+        if outputs is not None and b == batches[-1]:
+            rows = dump_rows(n_ent)
+            outputs.update(loss=last["loss"].detach().view(1), grad_ent_rows=rows,
+                           grad_ent=model.ent_emb.weight.grad[rows.to(dev)],
+                           grad_rel=model.rel_emb.weight.grad.clone())
         t0 = time.perf_counter()
         for _ in range(reps):
             e2e_step()
@@ -1017,23 +1088,27 @@ def run_c5(args, rank, world, dev):
     clocks = ClockSampler(dev.index) if rank == 0 else None
     if clocks is not None:
         clocks.start()
-    rec = measure_c5(args, dev, cpu_steps=0 if (args.no_cpu_baseline or rank != 0) else 3, batches=(4096, args.batch))
+    outputs = {} if args.dump_outputs and rank == 0 else None
+    rec = measure_c5(args, dev, cpu_steps=0 if (args.no_cpu_baseline or rank != 0) else 3, batches=(4096, args.batch),
+                     reps=args.steps, warm=args.warmup, outputs=outputs)
     clock_rec = clocks.stop() if clocks is not None else None
     if world > 1:
         dist.barrier()
     if rank == 0:
         b = rec["by_batch"][str(args.batch)]
         emit({"metric": C5_METRIC, "value": world * b["positives_per_s_fwd_bwd"], "unit": "positives/s",
-              "n_gpus": world, "steps": args.steps, "warmup": 3, "ms_per_step": b["fwd_bwd_ms"],
+              "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": b["fwd_bwd_ms"],
               "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
               "config": {"workload": c5_workload_text(args.batch),
                          "parallelism": "single GPU" if world == 1 else "%d independent replicas (no collective)" % world,
                          "l2_policy": "inputs larger than L2 (random rows of an 800 MB table)"},
               "e2e": {k: (v * world if k == "value" else v) for k, v in b["e2e"].items()},
-              "gpu_launches": 2 * max(3, min(args.steps, 10)), "clocks": clock_rec,
+              "gpu_launches": 2 * args.steps, "clocks": clock_rec,
               "roofline": dict(b["roofline_fwd_bwd"], kernel="margin_step_fast_kernel fwd + bwd", traffic=None,
                                forward_only=b["roofline_fwd"]),
               "parity": rec["parity"], "cpu_baseline": rec.get("cpu_baseline"), "by_batch": rec["by_batch"]})
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.destroy_process_group()
 

@@ -11,13 +11,15 @@ REF="${1:-/root/reference}"
 [ -d "$REF/torchkge" ] || { echo "make_ref: $REF/torchkge not found (nothing to do)"; exit 0; }
 TMP="$(mktemp -d)"
 trap 'rm -rf "$TMP"' EXIT
-cp -r "$REF" "$TMP/src"
+# copies keep the sources' read-only modes: make them writable, so that they can be replaced and removed
+cp -r "$REF" "$TMP/src" && chmod -R u+w "$TMP/src"
+if [ -d "$HERE/_ref" ]; then chmod -R u+w "$HERE/_ref"; fi
 rm -rf "$HERE/_ref"
 python -m pip install --quiet --no-index --no-build-isolation --no-deps --no-compile \
     --target "$HERE/_ref" "$TMP/src" 2>"$TMP/pip.log" || {
   # a plain copy of the package directory is the same thing for a pure-Python package
   echo "make_ref: pip install failed ($(tail -1 "$TMP/pip.log")); copying the package directory"
-  mkdir -p "$HERE/_ref" && cp -r "$REF/torchkge" "$HERE/_ref/torchkge"
+  mkdir -p "$HERE/_ref" && cp -r "$REF/torchkge" "$HERE/_ref/torchkge" && chmod -R u+w "$HERE/_ref"
 }
 python - <<PY
 import sys
